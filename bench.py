@@ -46,6 +46,10 @@ METRIC = 'aggregate detection FPS on synthetic 640x480 streams'
 UNIT = 'frames/s'
 W, H = 640, 480
 L2_BYTES = 126 * 1024 * 1024
+# watsor_b200.stream.share.Detection (72 bytes, include/watsor_b200.h: wb_detection)
+DETECTION_DTYPE = np.dtype({'names': ['label', 'zones', 'confidence', 'box'],
+                            'formats': ['<i4', ('<i4', (10,)), '<f8', ('<i4', (4,))],
+                            'offsets': [0, 4, 48, 56], 'itemsize': 72})
 
 
 def parse_args():
@@ -75,14 +79,21 @@ def parse_args():
     p.add_argument('--no-effects', action='store_true', help='skip the visual-effects record')
     p.add_argument('--min-seconds', type=float, default=1.0,
                    help='the *_long / e2e measurements run at least this long')
-    return p.parse_args()
+    p.add_argument('--dump-outputs', metavar='DIR',
+                   help='write what the last of the K timed steps returned (Detection rows and filter verdicts of '
+                        'every camera) to DIR/<name>.npy, as float64, to compare two builds output for output')
+    args = p.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        # the CPU arm times a few frames of the batch per step, so it has no per-step batch output to compare
+        p.error('--dump-outputs writes the outputs of the b200 arm; it cannot be combined with --impl reference')
+    return args
 
 
 # ------------------------------------------------------------------------------------------ inputs
 def load_model(kind):
     from watsor_b200.model import Model, synthetic_ssd_mobilenet_v1
     from tests.workload import v2_coco_model
-    blob = os.path.join(ROOT, 'models', '_ref', 'ssd_mobilenet_v1_shapes', 'b200.wb200')
+    blob = os.path.join(ROOT, 'oracle', '_ref', 'ssd_mobilenet_v1_shapes', 'b200.wb200')
     if kind == 'shapes' and os.path.isfile(blob):
         return Model.load(blob), 'ssd_mobilenet_v1 300x300, 3 classes, real weights (watsor/test/model/cpu.pb)'
     if kind == 'shapes':
@@ -388,6 +399,14 @@ class Arm:
         for i in range(max(0, n_steps - NS), n_steps):
             det.collect(i % NS, self.out_rows[i % NS], self.out_verd[i % NS])
 
+    def outputs(self, slot):
+        """What a caller of submit/collect received for the batch collected into `slot`, one row per camera: the
+        Detection[100] block field by field and the filter verdict bits, as float64 arrays (exact for every field)."""
+        rows = np.stack([np.frombuffer(bytes(r), dtype=DETECTION_DTYPE) for r in self.out_rows[slot]])
+        return {'detection_label': rows['label'], 'detection_zones': rows['zones'],
+                'detection_confidence': rows['confidence'], 'detection_box': rows['box'],
+                'filter_verdicts': np.stack(self.out_verd[slot])}
+
     def time_device(self, steps, first):
         """CUDA events on a torch stream fenced against the library's slot streams on both sides; max over ranks.
         The wall clock stops before the closing barrier (the NCCL barrier is not part of the loop)."""
@@ -447,6 +466,7 @@ class Arm:
         self.run_device_steps(warm, 0)
         launches = self.det.engine.last_launch_count()
         dev_ms, t_wall = self.time_device(args.steps, args.warmup)
+        self.last_outputs = self.outputs((args.steps - 1) % self.NS)
         out = {'value': world * C * args.steps / (dev_ms / 1e3), 'ms_per_step': dev_ms / args.steps,
                'launches_per_step': launches, 'wall_ms_per_step_device_loop': 1e3 * t_wall / args.steps,
                'prime_steps': self.prime_steps,
@@ -529,6 +549,8 @@ def main():
     if args.ingest == 'scatter' and world > 1:
         arm.enable_scatter()
     m = arm.measure()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, arm.last_outputs, rank if world > 1 else None)
     scatter = None
     if world > 1 and args.ingest == 'local' and not args.no_scatter:
         scatter = arm.measure_scatter(m['ms_per_step'])
@@ -627,6 +649,15 @@ def main():
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, arrays, rank=None):
+    """DIR/<name>.npy per array (DIR/<name>_rank<r>.npy with several ranks), float64."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if rank is not None:
+            name = '%s_rank%d' % (name, rank)
+        np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def measure_effects(args, local_rank, torch):

@@ -10,12 +10,15 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN_DIR = os.path.join(ROOT, 'tests', 'golden')
-MODEL_BLOB = os.path.join(ROOT, 'models', '_ref', 'ssd_mobilenet_v1_shapes', 'b200.wb200')
-REF_PB = '/root/reference/watsor/test/model/cpu.pb'
+# built by __graft_entry__.build() where a checkout of the original watsor project is readable
+# (oracle/reference_build.py); absent otherwise
+REF_BUILD = os.path.join(ROOT, 'oracle', '_ref')
+MODEL_BLOB = os.path.join(REF_BUILD, 'ssd_mobilenet_v1_shapes', 'b200.wb200')
+REF_PB = os.path.join(REF_BUILD, 'cpu.pb')
 
 
 def pytest_configure(config):
-    config.addinivalue_line('markers', 'gpu: needs a real B200 (run with `pytest -m gpu` under gpurun)')
+    config.addinivalue_line('markers', 'gpu: needs a real B200 (run with `pytest -m gpu`)')
 
 
 def has_gpu():
@@ -33,19 +36,36 @@ def golden():
 
 
 @pytest.fixture(scope='session')
-def shapes_model():
-    """The vendored 3-class SSD-MobileNet-v1 (real weights) as a compiled blob; built by
-    __graft_entry__.build() from /root/reference and carried to the GPU box by gpurun."""
+def real_shapes_model():
+    """The original project's 3-class SSD-MobileNet-v1 test model (watsor/test/model/cpu.pb, real weights) as a
+    compiled blob.  Its 22 MB of weights are not part of this repository: the tests that compare with vectors recorded
+    on those weights run where oracle/_ref/ has been built."""
     from watsor_b200.model import Model
     if not os.path.isfile(MODEL_BLOB):
-        pytest.skip('models/_ref blob missing (run __graft_entry__.build() where /root/reference exists)')
+        pytest.skip('oracle/_ref/ blob missing (__graft_entry__.build() found no checkout of the original project)')
     return Model.load(MODEL_BLOB)
+
+
+@pytest.fixture(scope='session')
+def shapes_model():
+    """The 3-class SSD-MobileNet-v1 for tests that compare two computations on the same model: the real weights where
+    oracle/_ref/ has been built, else the same architecture with seeded synthetic weights (as smoke() runs)."""
+    from watsor_b200.model import Model, synthetic_ssd_mobilenet_v1
+    if os.path.isfile(MODEL_BLOB):
+        return Model.load(MODEL_BLOB)
+    return synthetic_ssd_mobilenet_v1(num_classes=3, seed=1, score_thr=0.3)
 
 
 @pytest.fixture(scope='session')
 def shapes_oracle(shapes_model):
     from oracle.ssd_model import SsdModelOracle
     return SsdModelOracle(shapes_model)
+
+
+@pytest.fixture(scope='session')
+def real_shapes_oracle(real_shapes_model):
+    from oracle.ssd_model import SsdModelOracle
+    return SsdModelOracle(real_shapes_model)
 
 
 @pytest.fixture(scope='session')

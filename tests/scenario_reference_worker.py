@@ -5,7 +5,7 @@ runs in a separate *process* under `spawn`, the DetectionSieve filters confidenc
 labelled detections and the test passes when 100 have been seen.
 
 Run as a script in a fresh interpreter (tests/test_gpu_worker.py does) with the reference package on PYTHONPATH
-(`baseline/_ref`, installed by __graft_entry__.build() with pip from /root/reference): the detector module must
+(oracle/_ref/site, copied there by __graft_entry__.build() from a readable checkout): the detector module must
 bind to `watsor.stream.*` at import time, here and in the spawned child.
 
 Everything from `watsor.*` below is the reference's code; `create_object_detectors`, `ObjectDetector`,
@@ -65,7 +65,7 @@ def main(width=100, height=100, wanted=100, wait_s=90.0):
                                                          {get_coco_class(3).label: {'confidence': 50}}]})])]
     sieve = DetectionSieve('sieve', stop, log_queue, sieve_queue, frame_buffer, filters, RateLimiter())
     counter = ShapeCounter(Thread, 'counter', stop, log_queue, subscriber_queue, frame_buffer, latch)
-    model_path = os.path.join(ROOT, 'models', '_ref', 'ssd_mobilenet_v1_shapes')
+    model_path = os.path.join(ROOT, 'oracle', '_ref', 'ssd_mobilenet_v1_shapes')
     detectors = det_mod.create_object_detectors(Process, stop, log_queue, frame_queue, {artist.name: frame_buffer},
                                                 model_path)
     processes = [artist, sieve, counter] + detectors[:1]

@@ -7,6 +7,7 @@ import re
 import pytest
 
 from tests.conftest import ROOT, has_gpu
+from tests.reference_outputs import REFERENCE, Recorded, canon
 from watsor_b200 import _lib
 from watsor_b200.stream.share import BoundingBox, Detection, Frame, FrameBuffer, Header
 
@@ -22,22 +23,27 @@ def test_struct_layout_matches_reference_share_py():
             Header.detections.offset) == (0, 4, 8, 16, 24)
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference'), reason='reference tree not present')
-def test_struct_layout_equals_reference_module():
+def _layout(cls):
+    return [ctypes.sizeof(cls), [(f[0], getattr(cls, f[0]).offset) for f in cls._fields_]]
+
+
+def _reference_layouts():
     import importlib.util
     import sys
-    sys.path.insert(0, '/root/reference')
+    sys.path.insert(0, REFERENCE)
     try:
-        spec = importlib.util.spec_from_file_location('ref_share', '/root/reference/watsor/stream/share.py')
+        spec = importlib.util.spec_from_file_location('ref_share', os.path.join(REFERENCE, 'watsor', 'stream', 'share.py'))
         ref = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(ref)
     finally:
-        sys.path.remove('/root/reference')
+        sys.path.remove(REFERENCE)
+    return {name: _layout(getattr(ref, name)) for name in ('BoundingBox', 'Detection', 'Header')}
+
+
+def test_struct_layout_equals_reference_module():
+    theirs = Recorded('abi')('share.py struct layouts', _reference_layouts)
     for name in ('BoundingBox', 'Detection', 'Header'):
-        ours, theirs = globals()[name], getattr(ref, name)
-        assert ctypes.sizeof(ours) == ctypes.sizeof(theirs)
-        assert [(f[0], getattr(ours, f[0]).offset) for f in ours._fields_] == \
-               [(f[0], getattr(theirs, f[0]).offset) for f in theirs._fields_]
+        assert canon(_layout(globals()[name])) == theirs[name], name
 
 
 def test_frame_buffer_shared_memory_view():

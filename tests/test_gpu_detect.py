@@ -25,7 +25,7 @@ def test_device_name(detector):
     assert 'B200' in detector.device_name and len(detector.device_name.encode()) < 255
 
 
-def test_golden_cases_single_frame_protocol(detector, golden):
+def test_golden_cases_single_frame_protocol(detector, golden, real_shapes_model):
     """tensorflow_cpu.py:74-92 contract: detect(image_shape, image_np, detections) -> ms; all 100
     rows written; label/box ints exact (rounding ties tolerated and counted), confidence 1e-3."""
     flips = 0
@@ -57,7 +57,7 @@ def test_matches_oracle_on_fresh_artist_frames(detector, shapes_oracle, shapes_o
     assert total >= 20 and flips <= 2
 
 
-def test_batch_with_fused_porch_filters(detector, golden):
+def test_batch_with_fused_porch_filters(detector, golden, real_shapes_model):
     detector.configure_camera(0, 640, 480, PORCH_CONFIG)
     detector.configure_camera(1, 100, 100, None)
     detector.configure_camera(2, 320, 240, {'detect': [{'person': {'confidence': 50, 'area': 1}},

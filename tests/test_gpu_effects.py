@@ -138,7 +138,7 @@ def test_errors_are_loud(engine):
 
 
 def test_equal_to_the_reference_classes_installed_under_baseline_ref(engine):
-    """The UNMODIFIED reference package (baseline/_ref, installed by __graft_entry__.build(), travels to the GPU box)
+    """The UNMODIFIED reference package (oracle/_ref/site, copied by __graft_entry__.build() from a readable checkout)
     provides watsor.output.{blend,draw,copy}: run the reference's own effect chain on the CPU and the fused GPU effect
     on the same frame and rows.  watsor.filter.mask imports shapely (absent): an empty stand-in satisfies the import."""
     import sys
@@ -146,9 +146,9 @@ def test_equal_to_the_reference_classes_installed_under_baseline_ref(engine):
 
     from tests.conftest import ROOT
     from watsor_b200.output.effects import FusedEffects
-    ref_root = os.path.join(ROOT, 'baseline', '_ref')
+    ref_root = os.path.join(ROOT, 'oracle', '_ref', 'site')
     if not os.path.isfile(os.path.join(ref_root, 'watsor', 'output', 'draw.py')):
-        pytest.skip('baseline/_ref not installed')
+        pytest.skip('oracle/_ref/site not installed')
     saved = {k: v for k, v in sys.modules.items() if k == 'shapely' or k.startswith('shapely.') or
              k == 'watsor' or k.startswith('watsor.')}
     for k in saved:

@@ -80,7 +80,7 @@ def worker(rank, world, port, out):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(not os.path.isfile(MODEL_BLOB), reason='models/_ref blob missing')
+@pytest.mark.skipif(not os.path.isfile(MODEL_BLOB), reason='oracle/_ref/ blob missing')
 def test_two_rank_nccl_scatter_feeds_the_detector_in_place():
     import torch
     if torch.cuda.device_count() < 2:

@@ -87,7 +87,8 @@ def check_post(engine, oracle, enc, logits, cam=0, hw=(480, 640)):
     return n, mism
 
 
-def test_post_on_oracle_heads_golden_frames(engine, shapes_oracle, golden):
+def test_post_on_oracle_heads_golden_frames(engine, shapes_oracle, golden, real_shapes_model):
+    """The golden vectors were recorded on the real weights, which `engine` runs whenever they are built."""
     engine.set_camera(0, 640, 480)
     engine.set_camera(1, 100, 100)
     engine.set_camera(2, 320, 240)

@@ -1,8 +1,8 @@
 """The reference's own model test (ref: watsor/test/test_detect.py:28-77) with the reference's stream runtime
 (`watsor.stream`: FrameBuffer, StateLatch, Work / Spin, ReadDetectPublish Artist, ShapeCounter) and this repository's
 drop-in detector worker, sieve and filters on the real B200 back-end; the detector runs in a `Process` under
-`spawn`.  The reference package comes from `baseline/_ref` (pip-installed from /root/reference by
-__graft_entry__.build(); git-ignored, shipped to the GPU box by gpurun)."""
+`spawn`.  The reference package and model come from oracle/_ref/ (built by __graft_entry__.build() from a readable
+checkout of the original project, oracle/reference_build.py)."""
 import json
 import os
 import subprocess
@@ -13,12 +13,12 @@ import pytest
 from tests.conftest import MODEL_BLOB, ROOT
 
 pytestmark = pytest.mark.gpu
-REF_PKG = os.path.join(ROOT, 'baseline', '_ref')
+REF_PKG = os.path.join(ROOT, 'oracle', '_ref', 'site')
 
 
 @pytest.mark.skipif(not os.path.isfile(os.path.join(REF_PKG, 'watsor', 'stream', 'work.py')),
-                    reason='baseline/_ref (pip-installed reference package) is missing')
-@pytest.mark.skipif(not os.path.isfile(MODEL_BLOB), reason='models/_ref blob missing')
+                    reason='oracle/_ref/site (copy of the reference package) is missing')
+@pytest.mark.skipif(not os.path.isfile(MODEL_BLOB), reason='oracle/_ref/ blob missing')
 def test_shape_detection_reference_runtime_real_backend_spawned_process():
     env = dict(os.environ, PYTHONPATH=REF_PKG + os.pathsep + ROOT)
     out = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'scenario_reference_worker.py')], env=env,

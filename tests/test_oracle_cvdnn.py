@@ -28,17 +28,17 @@ def test_vectors_are_labelled_and_complete():
         assert z[key(*f) + '_enc'].shape == (1917, 4) and z[key(*f) + '_logits'].shape == (1917, 4)
 
 
-def test_blob_oracle_equals_opencv_dnn(shapes_oracle):
+def test_blob_oracle_equals_opencv_dnn(real_shapes_oracle):
     """oracle.raw_heads(pre) == OpenCV-dnn forward() of the reference's graph, <= 1e-4 (measured: 4e-5)."""
     z = np.load(NPZ)
     for f in FRAMES:
-        pre = shapes_oracle.preprocess(artist_frame(*f))
-        enc, lg = shapes_oracle.raw_heads(pre)
+        pre = real_shapes_oracle.preprocess(artist_frame(*f))
+        enc, lg = real_shapes_oracle.raw_heads(pre)
         assert np.abs(enc - z[key(*f) + '_enc']).max() <= TOL
         assert np.abs(lg - z[key(*f) + '_logits']).max() <= TOL
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_PB), reason='reference graph not present (GPU box)')
+@pytest.mark.skipif(not os.path.isfile(REF_PB), reason='oracle/_ref/cpu.pb not built')
 def test_live_opencv_run_reproduces_the_committed_vectors_and_the_graph_oracle():
     sys.path.insert(0, os.path.join(ROOT, 'tools'))
     from make_golden_cvdnn import cut_graph, run_cvdnn
@@ -60,14 +60,14 @@ def test_live_opencv_run_reproduces_the_committed_vectors_and_the_graph_oracle()
 
 @pytest.mark.gpu
 @pytest.mark.parametrize('precision', [0, 2], ids=['fp32-cuda-cores', 'fp32-3xtf32-tcgen05'])
-def test_gpu_heads_equal_opencv_dnn(shapes_model, shapes_oracle, precision):
+def test_gpu_heads_equal_opencv_dnn(real_shapes_model, real_shapes_oracle, precision):
     """The CUDA path against the independent executor directly (no oracle in between except the bit-exact resize)."""
     from watsor_b200.engine import Engine
     z = np.load(NPZ)
-    with Engine(shapes_model.to_blob(), device=0, max_batch=2, precision=precision) as e:
+    with Engine(real_shapes_model.to_blob(), device=0, max_batch=2, precision=precision) as e:
         for f in FRAMES:
             pre = e.preprocess([artist_frame(*f)])
-            assert np.array_equal(pre[0], shapes_oracle.preprocess(artist_frame(*f)))
+            assert np.array_equal(pre[0], real_shapes_oracle.preprocess(artist_frame(*f)))
             enc, lg, _ = e.backbone(pre)
             assert np.abs(enc[0] - z[key(*f) + '_enc']).max() <= 2e-4
             assert np.abs(lg[0] - z[key(*f) + '_logits']).max() <= 2e-4

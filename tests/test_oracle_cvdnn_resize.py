@@ -4,8 +4,8 @@ OWN node -- `Preprocessor/map/while/ResizeImage/resize/ResizeBilinear`, attribut
 and a constant size -- and runs it with its own kernel.  oracle.preprocess (the restatement every GPU parity test of
 the resize stage leans on, bit-exactly) must agree to float rounding at every size, up- and down-scaling.  Together
 with tests/test_oracle_cvdnn.py (convolutions) and tests/test_oracle_cvdnn_post.py (decode / NMS / top-100) this
-leaves no arithmetic stage of the graph pinned by the restatement's author alone.  CPU only; where /root/reference is
-absent the node is rebuilt with the same two attributes."""
+leaves no arithmetic stage of the graph pinned by the restatement's author alone.  CPU only; where oracle/_ref/cpu.pb
+is absent the node is rebuilt with the same two attributes."""
 import os
 
 import cv2

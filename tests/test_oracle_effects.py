@@ -1,7 +1,8 @@
 """oracle/effects.py against the reference's OWN effect classes (watsor/output/{copy,blend,draw}.py), imported from the
 read-only tree and run here on the same frames and Detection rows (SURVEY.md 8c: "outputs of the reference itself run
 here").  draw.py imports watsor.filter.mask, which imports shapely (absent): a bare stand-in module satisfies the
-import -- the effects never touch it.  CPU only; skipped where /root/reference is absent."""
+import -- the effects never touch it.  CPU only; the reference's frames are recorded (as digests) in
+tests/golden/reference/effects.json (tests/reference_outputs.py)."""
 import os
 import sys
 import types
@@ -14,12 +15,17 @@ import pytest
 from oracle import effects as oracle_fx
 from tests.fx_cases import random_alpha, random_rows
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not present')
+from tests.reference_outputs import REFERENCE as REF  # noqa: E402
+from tests.reference_outputs import Recorded, canon  # noqa: E402
+
+recorded = Recorded('effects')
 
 
 @pytest.fixture(scope='module')
 def ref():
+    if not REF:
+        yield None
+        return
     saved = {k: sys.modules.get(k) for k in ('shapely', 'shapely.geometry')}
     shapely, geometry = types.ModuleType('shapely'), types.ModuleType('shapely.geometry')
     geometry.Polygon = object
@@ -55,12 +61,27 @@ def test_copy_and_draw_chain(ref, size):
     for n_drawn in (0, 5, 30):
         img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
         rows = random_rows(rng, w, h, n_drawn)
-        header = as_header(ref, rows)
-        theirs = np.zeros_like(img)
-        ref.CopyImageEffect().apply(img, theirs, img.shape, header, header)
-        ref.DrawEffect().apply(img, theirs, img.shape, header, header)
+        theirs = recorded('copy+draw %dx%d %d' % (w, h, n_drawn), lambda: copy_and_draw(ref, img, rows))
         ours = oracle_fx.effect_chain(img, rows)
-        assert np.array_equal(theirs, ours), (size, n_drawn)
+        assert canon(ours) == theirs, (size, n_drawn)
+
+
+def copy_and_draw(ref, img, rows):
+    header = as_header(ref, rows)
+    theirs = np.zeros_like(img)
+    ref.CopyImageEffect().apply(img, theirs, img.shape, header, header)
+    ref.DrawEffect().apply(img, theirs, img.shape, header, header)
+    return theirs
+
+
+def blend_and_draw_with_contours(ref, config, img, rows):
+    """[after BlendEffect, after DrawEffectWithContours as well]."""
+    header = as_header(ref, rows)
+    theirs = np.zeros_like(img)
+    ref.BlendEffect(config).apply(img, theirs, img.shape, header, header)
+    blended = theirs.copy()
+    ref.DrawEffectWithContours(config).apply(img, theirs, img.shape, header, header)
+    return [blended, theirs]
 
 
 @pytest.mark.parametrize('size', [(320, 240), (200, 150)])
@@ -76,20 +97,22 @@ def test_blend_and_draw_with_contours_chain(ref, size):
             config = {'mask': path, 'width': w, 'height': h}
             img = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
             rows = random_rows(rng, w, h, 12, n_zones=nz)
-            header = as_header(ref, rows)
-            theirs = np.zeros_like(img)
-            ref.BlendEffect(config).apply(img, theirs, img.shape, header, header)
-            blended = theirs.copy()
-            ref.DrawEffectWithContours(config).apply(img, theirs, img.shape, header, header)
-            assert np.array_equal(blended, oracle_fx.effect_chain(img, rows, alpha, do_draw=False)), nz
-            assert np.array_equal(theirs, oracle_fx.effect_chain(img, rows, alpha)), nz
+            blended, theirs = recorded('blend+contours %dx%d %d' % (w, h, nz),
+                                       lambda: blend_and_draw_with_contours(ref, config, img, rows))
+            assert canon(oracle_fx.effect_chain(img, rows, alpha, do_draw=False)) == blended, nz
+            assert canon(oracle_fx.effect_chain(img, rows, alpha)) == theirs, nz
 
 
 def test_reference_draw_test_case(ref):
     """watsor/test/test_output.py:33-50: a 2x2 frame; the oracle must survive (and equal) the degenerate geometry."""
     rows = random_rows(np.random.default_rng(0), 2, 2, 2)
     img = np.zeros((2, 2, 3), np.uint8)
+    theirs = recorded('draw 2x2', lambda: draw_on_copy(ref, img, rows))
+    assert canon(oracle_fx.effect_chain(img, rows)) == theirs
+
+
+def draw_on_copy(ref, img, rows):
     header = as_header(ref, rows)
     theirs = img.copy()
     ref.DrawEffect().apply(img, theirs, img.shape, header, header)
-    assert np.array_equal(theirs, oracle_fx.effect_chain(img, rows))
+    return theirs

@@ -16,13 +16,13 @@ def test_artist_recipe_reproduces_committed_frames(golden):
         assert np.array_equal(img, load_golden_frame(case['name']))
 
 
-def test_blob_oracle_reproduces_golden_vectors(golden, shapes_oracle):
+def test_blob_oracle_reproduces_golden_vectors(golden, real_shapes_oracle):
     from oracle.ssd_graph import to_detections
     for case in golden['cases']:
         img = load_golden_frame(case['name'])
-        pre = shapes_oracle.preprocess(img)
+        pre = real_shapes_oracle.preprocess(img)
         assert hashlib.md5(pre.tobytes()).hexdigest() == case['pre_md5']      # pure numpy: bit exact
-        b, s, cl, n = shapes_oracle.postprocess(*shapes_oracle.raw_heads(pre))
+        b, s, cl, n = real_shapes_oracle.postprocess(*real_shapes_oracle.raw_heads(pre))
         assert n == case['num'] and [int(x) for x in cl[:n]] == case['classes']
         want_b = np.frombuffer(bytes.fromhex(case['boxes_f32']), '<f4').reshape(-1, 4)
         want_s = np.frombuffer(bytes.fromhex(case['scores_f32']), '<f4')
@@ -33,14 +33,14 @@ def test_blob_oracle_reproduces_golden_vectors(golden, shapes_oracle):
         assert rows[n] == (1, 0.0, 0, 0, 0, 0) and rows[99] == (1, 0.0, 0, 0, 0, 0)
 
 
-def test_oracle_finds_the_drawn_shapes(shapes_oracle):
+def test_oracle_finds_the_drawn_shapes(real_shapes_oracle):
     """The reference's behavioural pin (test_detect.py:28-77): on 100x100 Artist frames the
     detector reports labelled shapes with confidence >= 0.5; here additionally the right
     class at the right place."""
     hits = total = 0
     for frame in range(6):
         img, truth = artist_frame(100, 100, 5, frame, with_truth=True)
-        b, cl, s, n = shapes_oracle.run(img)
+        b, cl, s, n = real_shapes_oracle.run(img)
         from oracle.ssd_graph import to_detections
         rows = [r for r in to_detections(b, cl, s, img.shape)[:n] if r[1] >= 0.5]
         for shape, (x0, y0, x1, y1) in truth:
@@ -53,17 +53,17 @@ def test_oracle_finds_the_drawn_shapes(shapes_oracle):
     assert hits >= 0.7 * total, (hits, total)
 
 
-@pytest.mark.skipif(not os.path.isfile(REF_PB), reason='reference cpu.pb not present')
-def test_graph_oracle_and_blob_oracle_agree_bit_for_bit(shapes_oracle):
+@pytest.mark.skipif(not os.path.isfile(REF_PB), reason='oracle/_ref/cpu.pb not built')
+def test_graph_oracle_and_blob_oracle_agree_bit_for_bit(real_shapes_oracle):
     from oracle.ssd_graph import SsdGraphOracle
     og = SsdGraphOracle(REF_PB)
     img = np.random.default_rng(3).integers(0, 256, (240, 320, 3), dtype=np.uint8)
     pre = og.preprocess(img)
-    assert np.array_equal(pre, shapes_oracle.preprocess(img))
+    assert np.array_equal(pre, real_shapes_oracle.preprocess(img))
     e1, l1 = og.raw_heads(pre)
-    e2, l2 = shapes_oracle.raw_heads(pre)
+    e2, l2 = real_shapes_oracle.raw_heads(pre)
     assert np.array_equal(e1, e2) and np.array_equal(l1, l2)
-    for a, b in zip(og.postprocess(e1, l1), shapes_oracle.postprocess(e2, l2)):
+    for a, b in zip(og.postprocess(e1, l1), real_shapes_oracle.postprocess(e2, l2)):
         assert np.array_equal(a, b)
 
 

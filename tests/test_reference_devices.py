@@ -1,15 +1,15 @@
 """`b200_gpus()` against the reference's own `cuda_gpus()` (watsor/detection/devices.py:28-77), run here with
 stand-in `pycuda.driver` / `watsor.detection.tensorrt_gpu` modules that only report a device count: same devices
 in the same order, same TypeError, for every combination of CUDA_DEVICE, ~/.cuda_device and device count.
-CPU only; skipped where /root/reference is absent."""
-import os
+CPU only; the reference's answers are recorded in tests/golden/reference/devices.json (tests/reference_outputs.py)."""
 import sys
 import types
 
 import pytest
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not present')
+from tests.reference_outputs import REFERENCE, Recorded, canon
+
+recorded = Recorded('devices')
 
 
 @pytest.fixture()
@@ -25,21 +25,23 @@ def both(monkeypatch):
     trt.TensorRTObjectDetector = type('TensorRTObjectDetector', (), {})
     for name, mod in (('pycuda', pycuda), ('pycuda.driver', driver), ('watsor.detection.tensorrt_gpu', trt)):
         monkeypatch.setitem(sys.modules, name, mod)
-    monkeypatch.syspath_prepend(REF)
-    from watsor.detection.devices import cuda_gpus
+    cuda_gpus = None
+    if REFERENCE:
+        monkeypatch.syspath_prepend(REFERENCE)
+        from watsor.detection.devices import cuda_gpus
     from watsor_b200 import _lib
     from watsor_b200.detection.devices import b200_gpus
     monkeypatch.setattr(_lib, 'device_count', lambda: count['n'])
 
-    def run(n):
+    def call(gen):
+        try:
+            return [d for d, _ in gen()]
+        except TypeError as e:
+            return 'TypeError: %s' % e
+
+    def run(n, key):
         count['n'] = n
-        out = []
-        for gen in (cuda_gpus, b200_gpus):
-            try:
-                out.append([d for d, _ in gen()])
-            except TypeError as e:
-                out.append('TypeError: %s' % e)
-        return out
+        return recorded(key, lambda: call(cuda_gpus)), canon(call(b200_gpus))
     yield run
     for name in [m for m in sys.modules if m == 'watsor' or m.startswith('watsor.')]:
         sys.modules.pop(name, None)
@@ -60,7 +62,7 @@ def test_same_devices_as_the_reference_generator(both, monkeypatch, tmp_path, n,
             (tmp_path / '.cuda_device').write_text(dotfile)
     else:
         monkeypatch.delenv('HOME', raising=False)
-    theirs, ours = both(n)
+    theirs, ours = both(n, repr((n, env, dotfile, home)))
     assert ours == theirs, (n, env, dotfile, home)
     if n == 0:
         assert ours == []

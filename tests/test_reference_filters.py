@@ -3,7 +3,8 @@
 as they are.  MaskFilter needs shapely, which is not installed: it is imported with a stand-in `shapely.geometry`
 whose `Polygon.intersects` is the oracle's exact integer geometry, so this pins the reference's control flow --
 alpha threshold, contour extraction and ordering, per-class zone lists, the order and cap of `zones[]` writes --
-but not GEOS itself (that gap is stated in DESIGN.md section 5).  CPU only; skipped where /root/reference is absent."""
+but not GEOS itself (that gap is stated in DESIGN.md section 5).  CPU only; the reference's verdicts are recorded in
+tests/golden/reference/filters.json (tests/reference_outputs.py)."""
 import os
 import sys
 import types
@@ -14,9 +15,9 @@ import pytest
 
 from oracle.filters import AreaOracle, ConfidenceOracle, Det, MaskOracle, rect_intersects_polygon
 from tests.conftest import PORCH_CONFIG
+from tests.reference_outputs import REFERENCE, Recorded
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not present')
+recorded = Recorded('filters')
 
 
 class _StandInPolygon:
@@ -35,13 +36,16 @@ class _StandInPolygon:
 
 @pytest.fixture(scope='module')
 def ref():
+    if not REFERENCE:
+        yield None
+        return
     saved = {k: sys.modules.get(k) for k in ('shapely', 'shapely.geometry')}
     shapely = types.ModuleType('shapely')
     geometry = types.ModuleType('shapely.geometry')
     geometry.Polygon = _StandInPolygon
     shapely.geometry = geometry
     sys.modules['shapely'], sys.modules['shapely.geometry'] = shapely, geometry
-    sys.path.insert(0, REF)
+    sys.path.insert(0, REFERENCE)
     try:
         from watsor.filter.area import AreaFilter
         from watsor.filter.confidence import ConfidenceFilter
@@ -50,7 +54,7 @@ def ref():
         yield types.SimpleNamespace(AreaFilter=AreaFilter, ConfidenceFilter=ConfidenceFilter, MaskFilter=MaskFilter,
                                     BoundingBox=BoundingBox, Detection=Detection)
     finally:
-        sys.path.remove(REF)
+        sys.path.remove(REFERENCE)
         for k, v in saved.items():
             if v is None:
                 sys.modules.pop(k, None)
@@ -58,7 +62,7 @@ def ref():
                 sys.modules[k] = v
 
 
-def random_dets(rng, ref, w, h, n):
+def random_dets(rng, w, h, n):
     out = []
     for r in range(n):
         x0, x1 = (int(v) for v in rng.integers(-5, w + 5, 2))
@@ -69,8 +73,34 @@ def random_dets(rng, ref, w, h, n):
             x1, y1 = x0, y0
         label = int(rng.integers(0, 6))
         conf = [0.5, 0.25, 0.75, float(np.float32(rng.random())), float(rng.random())][r % 5]
-        rd = ref.Detection(label=label, confidence=conf, bounding_box=ref.BoundingBox(x0, y0, x1, y1))
-        out.append((rd, Det(label, conf, (x0, y0, x1, y1))))
+        out.append(Det(label, conf, (x0, y0, x1, y1)))
+    return out
+
+
+def verdicts(ref, filt, dets):
+    """The reference filter `filt` on each Det: one character per verdict ('T' / 'F', both bools) and the zones it
+    wrote, by index and without trailing zeros, where any are non-zero."""
+    marks, zones = [], {}
+    for i, d in enumerate(dets):
+        rd = ref.Detection(label=d.label, confidence=d.confidence,
+                           bounding_box=ref.BoundingBox(d.x_min, d.y_min, d.x_max, d.y_max))
+        v = filt(rd)
+        assert isinstance(v, bool)
+        marks.append('T' if v else 'F')
+        z = list(rd.zones)
+        while z and z[-1] == 0:
+            z.pop()
+        if z:
+            zones[str(i)] = ','.join(map(str, z))
+    return {'verdicts': ''.join(marks), 'zones': zones}
+
+
+def unpack(rec):
+    """[(verdict, zones)] per Det from what `verdicts` recorded."""
+    out = []
+    for i, m in enumerate(rec['verdicts']):
+        z = [int(v) for v in rec['zones'][str(i)].split(',')] if str(i) in rec['zones'] else []
+        out.append((m == 'T', z + [0] * (10 - len(z))))
     return out
 
 
@@ -83,14 +113,15 @@ def test_confidence_and_area_oracles_equal_the_reference_classes(ref, seed):
                       {'car': {'confidence': 50, 'area': 10}},
                       {'bicycle': {'confidence': 25, 'area': 0}},
                       {'motorcycle': {'confidence': 75, 'area': 100}}]}
-    rc, ra = ref.ConfidenceFilter(cfg), ref.AreaFilter(cfg)
     oc, oa = ConfidenceOracle(cfg), AreaOracle(cfg)
-    for rd, od in random_dets(rng, ref, w, h, 1500):
-        assert rc(rd) == oc(od) and ra(rd) == oa(od), od.key()
-    # the full-frame box is exactly 100 % (area.py:18, :24-26)
-    full = (ref.Detection(label=4, confidence=0.75, bounding_box=ref.BoundingBox(0, 0, w - 1, h - 1)),
-            Det(4, 0.75, (0, 0, w - 1, h - 1)))
-    assert ra(full[0]) is True and oa(full[1]) is True and rc(full[0]) is True and oc(full[1]) is True
+    # the last one is the full-frame box, exactly 100 % (area.py:18, :24-26)
+    dets = random_dets(rng, w, h, 1500) + [Det(4, 0.75, (0, 0, w - 1, h - 1))]
+    rc = unpack(recorded('confidence/%d' % seed, lambda: verdicts(ref, ref.ConfidenceFilter(cfg), dets)))
+    ra = unpack(recorded('area/%d' % seed, lambda: verdicts(ref, ref.AreaFilter(cfg), dets)))
+    assert len(rc) == len(ra) == len(dets)
+    for od, (c, _), (a, _) in zip(dets, rc, ra):
+        assert c == oc(od) and a == oa(od), od.key()
+    assert ra[-1][0] is True and oa(dets[-1]) is True and rc[-1][0] is True and oc(dets[-1]) is True
 
 
 def _random_alpha(rng, w, h):
@@ -122,31 +153,45 @@ def test_mask_oracle_equals_reference_control_flow(ref, seed):
         try:
             n_zones = len(MaskOracle(base).polygons)
         except (AssertionError, ZeroDivisionError):
-            with pytest.raises((ValueError, ZeroDivisionError)):
-                ref.MaskFilter(base)                             # the reference rejects the same masks
+            # the reference rejects the same masks
+            assert recorded('mask/%d/rejects' % seed, lambda: raised(ref.MaskFilter, base)) in \
+                ('ValueError', 'ZeroDivisionError')
             return
         zones_b = sorted(int(z) for z in rng.choice(np.arange(1, n_zones + 1), size=int(rng.integers(1, n_zones + 1)),
                                                     replace=False))
         cfg = {'width': w, 'height': h, 'mask': tmp.name,
                'detect': [{'person': {'zones': []}}, {'bicycle': {'zones': zones_b}}, {'car': {'zones': [n_zones]}}]}
-        rm, om = ref.MaskFilter(cfg), MaskOracle(cfg)
+        om = MaskOracle(cfg)
+        bad_zone = {**cfg, 'detect': [{'person': {'zones': [n_zones + 1]}}]}
+        assert recorded('mask/%d/bad_zone' % seed, lambda: raised(ref.MaskFilter, bad_zone)) == 'AssertionError'
         with pytest.raises(AssertionError):
-            ref.MaskFilter({**cfg, 'detect': [{'person': {'zones': [n_zones + 1]}}]})
-        with pytest.raises(AssertionError):
-            MaskOracle({**cfg, 'detect': [{'person': {'zones': [n_zones + 1]}}]})
+            MaskOracle(bad_zone)
+        dets = random_dets(rng, w, h, 600)
+        theirs = unpack(recorded('mask/%d' % seed, lambda: verdicts(ref, ref.MaskFilter(cfg), dets)))
+        assert len(theirs) == len(dets)
     finally:
         tmp.close()
         os.unlink(tmp.name)
-    for rd, od in random_dets(rng, ref, w, h, 600):
-        assert rm(rd) == om(od) and list(rd.zones) == od.zones, od.key()
+    for od, (verdict, zones) in zip(dets, theirs):
+        assert verdict == om(od) and zones == od.zones, od.key()
+
+
+def raised(fn, *args):
+    """The name of the exception `fn(*args)` raises, None when it returns."""
+    try:
+        fn(*args)
+    except Exception as e:
+        return type(e).__name__
+    return None
 
 
 def test_porch_mask_reference_control_flow(ref):
-    rm, om = ref.MaskFilter(PORCH_CONFIG), MaskOracle(PORCH_CONFIG)
-    rng = np.random.default_rng(3)
+    om = MaskOracle(PORCH_CONFIG)
+    dets = random_dets(np.random.default_rng(3), 640, 480, 3000)
+    theirs = unpack(recorded('porch', lambda: verdicts(ref, ref.MaskFilter(PORCH_CONFIG), dets)))
+    assert len(theirs) == len(dets)
     hits = 0
-    for rd, od in random_dets(rng, ref, 640, 480, 3000):
-        got = rm(rd)
-        assert got == om(od) and list(rd.zones) == od.zones, od.key()
+    for od, (got, zones) in zip(dets, theirs):
+        assert got == om(od) and zones == od.zones, od.key()
         hits += got
     assert 300 < hits < 2900

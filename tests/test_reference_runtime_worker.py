@@ -11,8 +11,9 @@ from tests.conftest import ROOT
 
 
 def reference_path():
-    for p in ('/root/reference', os.path.join(ROOT, 'baseline', '_ref')):
-        if os.path.isfile(os.path.join(p, 'watsor', 'stream', 'work.py')):
+    from oracle.reference_build import find_reference
+    for p in (find_reference(), os.path.join(ROOT, 'oracle', '_ref', 'site')):
+        if p and os.path.isfile(os.path.join(p, 'watsor', 'stream', 'work.py')):
             return p
     return None
 

@@ -2,7 +2,7 @@
 TrackFilter (watsor/filter/track.py:29-149) and the sieve write-back (watsor/filter/sieve.py:21-52).
 
 Pinned by (a) the reference's known answers (watsor/test/test_filter.py:76-96), (b) the reference's TrackFilter
-itself, imported from /root/reference when present, (c) the oracle restatement, (d) the CPython interpreter for
+itself, its results recorded in tests/golden/reference/tracker.json (tests/reference_outputs.py), (c) the oracle restatement, (d) the CPython interpreter for
 the set iteration orders the reference leaks into its results.  No GPU involved."""
 import ctypes
 import os
@@ -16,7 +16,10 @@ from oracle.filters import Det, TrackOracle
 from watsor_b200 import _lib
 from watsor_b200.stream.share import MAX_DETECTIONS, BoundingBox, Detection
 
-REF = '/root/reference'
+from tests.reference_outputs import REFERENCE as REF  # noqa: E402
+from tests.reference_outputs import Recorded  # noqa: E402
+
+recorded = Recorded('tracker')
 
 
 class NativeTracker:
@@ -146,11 +149,14 @@ def test_native_tracker_equals_oracle(seed, sens, hist, per_label, labels, zone_
         assert [key(d) for d in got] == [d.key() for d in exp], f
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not present')
-@pytest.mark.parametrize('seed,sens,hist,per_label,labels,zone_ids',
-                         [(11, 1, 2, 3, 2, 3), (12, 5, 10, 10, 3, 12), (13, 2, 4, 14, 1, 9), (14, 3, 6, 7, 5, 5)])
-def test_native_tracker_equals_reference_trackfilter(seed, sens, hist, per_label, labels, zone_ids):
-    """The reference's own TrackFilter (watsor/filter/track.py), imported from the read-only tree."""
+def frame_digest(sa, dets):
+    """A tracker's answer for one frame, (sa, the kept detections' keys), as a short digest."""
+    import hashlib
+    return hashlib.sha256(repr((sa, [key(d) for d in dets])).encode()).hexdigest()[:16]
+
+
+def reference_trackfilter(frames, sens, hist):
+    """frame_digest() of the reference's TrackFilter on every frame."""
     sys.path.insert(0, REF)
     try:
         from watsor.filter.track import TrackFilter as RefTrackFilter
@@ -158,20 +164,32 @@ def test_native_tracker_equals_reference_trackfilter(seed, sens, hist, per_label
         from watsor.stream.share import Detection as RefDetection
     finally:
         sys.path.remove(REF)
-    rng = random.Random(seed)
-    frames = random_frames(rng, 150, per_label, labels, zone_ids)
-    nat, ref = NativeTracker(sens, hist), RefTrackFilter(sensitivity=sens, history=hist)
-    for f, dets in enumerate(frames):
-        got, sa = nat([mk(*d) for d in dets])
+    ref, out = RefTrackFilter(sensitivity=sens, history=hist), []
+    for dets in frames:
         rdets = []
         for l, c, b, z in dets:
             d = RefDetection(label=l, confidence=c, bounding_box=RefBox(*b))
             for i, zz in enumerate(z):
                 d.zones[i] = zz
             rdets.append(d)
-        exp, sa_r = ref(rdets)
-        assert sa == sa_r, f
-        assert [key(d) for d in got] == [key(d) for d in exp], f
+        exp, sa = ref(rdets)
+        assert isinstance(sa, bool)
+        out.append(frame_digest(sa, exp))
+    return out
+
+
+@pytest.mark.parametrize('seed,sens,hist,per_label,labels,zone_ids',
+                         [(11, 1, 2, 3, 2, 3), (12, 5, 10, 10, 3, 12), (13, 2, 4, 14, 1, 9), (14, 3, 6, 7, 5, 5)])
+def test_native_tracker_equals_reference_trackfilter(seed, sens, hist, per_label, labels, zone_ids):
+    """The reference's own TrackFilter (watsor/filter/track.py), frame by frame."""
+    rng = random.Random(seed)
+    frames = random_frames(rng, 150, per_label, labels, zone_ids)
+    theirs = recorded('trackfilter %d' % seed, lambda: reference_trackfilter(frames, sens, hist))
+    assert len(theirs) == len(frames)
+    nat = NativeTracker(sens, hist)
+    for f, dets in enumerate(frames):
+        got, sa = nat([mk(*d) for d in dets])
+        assert frame_digest(sa, got) == theirs[f], f
 
 
 def test_sieve_rows_writes_back_and_zero_fills():
@@ -325,37 +343,43 @@ for n in (64, 100):
         lib.wb_debug_argsort(a.ctypes.data, n, out)
         res['argsort_cases'] += 1
         res['argsort_mismatch'] += int(list(out) != list(np.argsort(a.astype(np.float64))))
-res['track_diverging'] = -1
+# tie-heavy tracking: frame_digest() of every frame of 5 x 8 sequences, by the native tracker and -- where the original
+# project is readable -- by its TrackFilter, both under this interpreter's scalar numpy
+from tests.test_tracker import TIE_HEAVY, NativeTracker, frame_digest, mk
 if %(with_ref)r:
-    from tests.test_tracker import NativeTracker, mk, key
     sys.path.insert(0, %(ref)r)
     from watsor.filter.track import TrackFilter
     from watsor.stream.share import BoundingBox, Detection
-    bad = 0
-    for max_n, grid in ((12, 6), (24, 20), (40, 6), (40, 60), (100, 30)):
-        for seed in range(8):
-            r = random.Random(seed)
-            nat, ref = NativeTracker(2, 4), TrackFilter(sensitivity=2, history=4)
-            for f in range(40):
-                dets = []
-                for _ in range(r.randint(0, max_n)):
-                    x, y = r.randint(0, grid), r.randint(0, grid)
-                    dets.append((r.randint(1, 2), 0.5 + 0.01 * r.randint(0, 40), (x, y, x + r.choice([2, 4]), y + r.choice([2, 4])),
-                                 [r.randint(1, 12)] if r.random() < 0.5 else []))
-                got, _ = nat([mk(*d) for d in dets])
-                rd = []
-                for l, c, b, z in dets:
-                    d = Detection(label=l, confidence=c, bounding_box=BoundingBox(*b))
-                    for i, zz in enumerate(z):
-                        d.zones[i] = zz
-                    rd.append(d)
-                exp, _ = ref(rd)
-                if [key(d) for d in got] != [key(d) for d in exp]:
-                    bad += 1
-                    break
-    res['track_diverging'] = bad
+res['native'], res['reference'] = {}, {}
+for max_n, grid in TIE_HEAVY:
+    for seed in range(8):
+        r = random.Random(seed)
+        name = 'tie-heavy max_n=%%d grid=%%d seed=%%d' %% (max_n, grid, seed)
+        nat = NativeTracker(2, 4)
+        ref = TrackFilter(sensitivity=2, history=4) if %(with_ref)r else None
+        res['native'][name], res['reference'][name] = [], []
+        for f in range(40):
+            dets = []
+            for _ in range(r.randint(0, max_n)):
+                x, y = r.randint(0, grid), r.randint(0, grid)
+                dets.append((r.randint(1, 2), 0.5 + 0.01 * r.randint(0, 40), (x, y, x + r.choice([2, 4]), y + r.choice([2, 4])),
+                             [r.randint(1, 12)] if r.random() < 0.5 else []))
+            got, sa = nat([mk(*d) for d in dets])
+            res['native'][name].append(frame_digest(sa, got))
+            if ref is None:
+                continue
+            rd = []
+            for l, c, b, z in dets:
+                d = Detection(label=l, confidence=c, bounding_box=BoundingBox(*b))
+                for i, zz in enumerate(z):
+                    d.zones[i] = zz
+                rd.append(d)
+            exp, sa = ref(rd)
+            assert isinstance(sa, bool)
+            res['reference'][name].append(frame_digest(sa, exp))
 print(json.dumps(res))
 '''
+TIE_HEAVY = ((12, 6), (24, 20), (40, 6), (40, 60), (100, 30))      # (max detections per frame, coordinate grid)
 
 
 def test_argsort_and_tie_heavy_tracking_match_numpy_scalar_sort():
@@ -363,7 +387,7 @@ def test_argsort_and_tie_heavy_tracking_match_numpy_scalar_sort():
     on AVX2 / AVX-512 machines, so the comparison runs in a child interpreter with those code paths disabled
     (NPY_DISABLE_CPU_FEATURES) -- the arithmetic of the reference's pinned numpy 1.23.  With it, the tie-heavy
     tracking sequences (tiny coordinate grids, up to 100 detections of a label per frame) equal the reference's
-    TrackFilter on every frame."""
+    TrackFilter on every frame (its answers recorded in tests/golden/reference/tracker.json)."""
     import json
     import subprocess
     from numpy._core._multiarray_umath import __cpu_features__ as feats
@@ -374,7 +398,7 @@ def test_argsort_and_tie_heavy_tracking_match_numpy_scalar_sort():
     if simd:
         env['NPY_DISABLE_CPU_FEATURES'] = ' '.join(simd)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    script = _SCALAR_NUMPY_SCRIPT % {'root': root, 'ref': REF, 'with_ref': os.path.isdir(REF)}
+    script = _SCALAR_NUMPY_SCRIPT % {'root': root, 'ref': REF, 'with_ref': bool(REF)}
     p = subprocess.run([sys.executable, '-c', script], env=env, capture_output=True, text=True, timeout=300)
     if p.returncode != 0 and 'NPY_DISABLE_CPU_FEATURES' in p.stderr:
         pytest.skip('numpy refused to disable its SIMD dispatch: ' + p.stderr.strip().splitlines()[-1])
@@ -382,4 +406,9 @@ def test_argsort_and_tie_heavy_tracking_match_numpy_scalar_sort():
     res = json.loads(p.stdout.strip().splitlines()[-1])
     assert res['unstable_seen'] > 0                              # the cases do exercise non-stable orders
     assert res['argsort_mismatch'] == 0, res
-    assert res['track_diverging'] in (0, -1), res
+    assert len(res['native']) == 5 * 8
+    for name, ours in res['native'].items():
+        theirs = recorded(name, lambda: res['reference'][name])
+        assert len(ours) == len(theirs) == 40, name
+        diverging = [f for f, (a, b) in enumerate(zip(ours, theirs)) if a != b]
+        assert not diverging, (name, 'first diverging frame', diverging[0])

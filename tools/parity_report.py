@@ -13,6 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch  # noqa: E402
 
+from oracle.reference_build import MODEL_BLOB  # noqa: E402
 from oracle.ssd_graph import to_detections  # noqa: E402
 from oracle.ssd_model import SsdModelOracle  # noqa: E402
 from tests.artist import artist_frame  # noqa: E402
@@ -24,7 +25,7 @@ from watsor_b200.stream.share import Detection  # noqa: E402
 n_frames = int(sys.argv[1]) if len(sys.argv) > 1 else 120
 rnd = sys.argv[2] if len(sys.argv) > 2 else 'r01'
 torch.set_num_threads(16)
-model = Model.load(os.path.join(ROOT, 'models', '_ref', 'ssd_mobilenet_v1_shapes', 'b200.wb200'))
+model = Model.load(MODEL_BLOB)
 o32, o64 = SsdModelOracle(model), SsdModelOracle(model, dtype=np.float64)
 sizes = [(100, 100), (320, 240), (640, 480), (1920, 1080)]
 frames = [artist_frame(*sizes[i % 4], cam=100 + i % 7, frame=i) for i in range(n_frames)]

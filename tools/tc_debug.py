@@ -4,11 +4,12 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from watsor_b200.engine import Engine
 from watsor_b200.model import Model, OP_HEAD, OP_NAMES
+from oracle.reference_build import MODEL_BLOB
 from oracle.ssd_model import SsdModelOracle
 from tests.artist import artist_frame
 
 prec = [int(x) for x in sys.argv[1].split(',')] if len(sys.argv) > 1 else [3, 2, 1]
-m = Model.load('models/_ref/ssd_mobilenet_v1_shapes/b200.wb200')
+m = Model.load(MODEL_BLOB)
 o = SsdModelOracle(m)
 imgs = [artist_frame(640, 480, 0, f) for f in range(3)]
 pres = np.stack([o.preprocess(i) for i in imgs])

@@ -6,12 +6,12 @@ Runs the backbone up to a chosen layer, then reads the clock64() stamps the last
 kernel left (see WB_STAMP in tc_common.cuh) and prints them relative to the kernel start, in cycles.
 """
 import ctypes
-import glob
 import sys
 
 import numpy as np
 
 sys.path.insert(0, '.')
+from oracle.reference_build import MODEL_BLOB  # noqa: E402
 from watsor_b200.engine import Engine  # noqa: E402
 
 SLOTS, ITERS = 12, 64
@@ -32,7 +32,7 @@ def dump(e, fn, names, start_kind, n_it):
 
 
 def main():
-    blob = open(glob.glob('models/_ref/*/b200.wb200')[0], 'rb').read()
+    blob = open(MODEL_BLOB, 'rb').read()
     e = Engine(blob, max_batch=8, precision=2)
     pre = np.random.default_rng(0).uniform(-1, 1, (8, 300, 300, 3)).astype(np.float32)
     for rep in range(3):
